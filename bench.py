@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- surround-BEV frame-sets/s on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the fused BEV path over one batch of synthetic frame-sets:
@@ -144,6 +144,26 @@ def algorithmic_bytes(eng, masks, w):
     return int(src), int(canvas)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, canvases, seed=0):
+    """Write the canvases of the last timed step (uint8 [n][BH][BW][3]) under `path` for output-by-output comparison of
+    two builds: all of them as canvases.npy (float32) when that fits in DUMP_BYTES, otherwise a fixed, seeded sample
+    of whole canvas rows as canvas_rows.npy (float32 [k][BW][3]) with their (canvas, row) numbers in
+    canvas_row_index.npy (float64 [k][2])."""
+    os.makedirs(path, exist_ok=True)
+    canvases = np.asarray(canvases)
+    n, h, w = canvases.shape[:3]
+    if canvases.size * 4 <= DUMP_BYTES:
+        np.save(os.path.join(path, "canvases.npy"), canvases.astype(np.float32))
+        return
+    k = (DUMP_BYTES - (1 << 20)) // (w * 3 * 4)                     # 1 MB left for the index and the .npy headers
+    rows = np.sort(np.random.default_rng(seed).choice(n * h, k, replace=False))
+    np.save(os.path.join(path, "canvas_rows.npy"), canvases.reshape(n * h, w, 3)[rows].astype(np.float32))
+    np.save(os.path.join(path, "canvas_row_index.npy"), np.stack([rows // h, rows % h], 1).astype(np.float64))
+
+
 # ----------------------------------------------------------------------------- clocks
 class ClockSampler(threading.Thread):
     REASONS = {0x8: "hw_slowdown", 0x40: "hw_thermal_slowdown", 0x20: "sw_thermal_slowdown", 0x4: "sw_power_cap",
@@ -261,7 +281,11 @@ def main():
                          "'cameras-p2p' = the fused kernel stores slabs into the owning rank over NVLink, canvases stay sharded)")
     ap.add_argument("--workload", default="cfg4", choices=sorted(ALT_WORKLOADS),
                     help="cfg4 (default) is the headline; the others are secondary measurements of BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the canvases of the last timed step (rank 0) to DIR/*.npy as float32")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     w = dict(WORKLOAD, **ALT_WORKLOADS[a.workload])
     if a.batch:
         w["batch"] = a.batch
@@ -313,9 +337,10 @@ def main():
             ref(*sets[0])
         t0 = time.perf_counter()
         for _ in range(a.steps):
-            for s in sets:
-                ref(*s)
+            last = [ref(*s) for s in sets]
         dt = time.perf_counter() - t0
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, np.stack(last))
         v = a.steps * per_step / dt
         line = {"impl": "reference", "metric": metric, "value": v, "unit": unit, "n_gpus": a.gpus, "steps": a.steps,
                 "warmup": a.warmup, "ms_per_step": dt / a.steps * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -405,6 +430,7 @@ def main():
     e1.record(stream)
     barrier()
     ms = e0.elapsed_time(e1)
+    last = (d_own if p2p else d_out).cpu().numpy() if a.dump_outputs and rank == 0 else None   # before any untimed step
     launches = eng.ctx.launches - l0
     # keep the GPU under the same load a little longer so the clock sampler sees it (untimed)
     t_end = time.time() + 1.0
@@ -538,6 +564,8 @@ def main():
             line["cpu_baseline"] = {"value": v, "unit": unit, "cores": cores, "kind": "port",
                                     "sample": sample + f"; os.cpu_count()={os.cpu_count()}",
                                     "frame_set_parallel": cpu_parallel}
+        if last is not None:
+            dump_outputs(a.dump_outputs, last)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

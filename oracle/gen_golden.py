@@ -1,4 +1,4 @@
-"""Generate tests/golden/{fixtures.npz,golden.json} from the UNMODIFIED reference.
+"""Generate tests/golden/{fixtures.npz,golden.json,reference_samples.npz} from the UNMODIFIED reference.
 
 TEST INFRASTRUCTURE ONLY.  Run in the build container (where /root/reference
 exists):  ``python -m oracle.gen_golden``.  It imports the reference's own
@@ -12,7 +12,11 @@ runs them on the reference's own data/ images and records
     recorded too so a decoder change is detected);
   * golden.json  -- SHA-256 prefixes (16 hex) of every output of the reference on
     those inputs: maps, masks, per-camera warps, BevGenerator at all flag
-    combinations and at the rescaled configs of BASELINE.json.
+    combinations and at the rescaled configs of BASELINE.json;
+  * reference_samples.npz -- values of the reference's BevGenerator(blend=True,
+    balance=True) canvas (with car) and of each camera's BEV map at a fixed, seeded
+    set of canvas pixels, so that tests compare against the reference's own numbers
+    without the reference being installed.
 """
 from __future__ import annotations
 
@@ -163,6 +167,19 @@ def main():
     with open(os.path.join(OUT, "golden.json"), "w") as f:
         json.dump(gold, f, indent=1, sort_keys=True)
     print(json.dumps(gold, indent=1, sort_keys=True))
+    write_reference_samples(F, car)
+
+
+def write_reference_samples(frames, car, n_pixels=4096, seed=2024):
+    """tests/golden/reference_samples.npz: the reference's blended, balanced canvas (with car) and every camera's BEV
+    map (map1: integer source coordinates) at n_pixels canvas pixels drawn with a fixed seed."""
+    b = RL.make_bev(blend=True, balance=True)
+    bev = b(*frames, car)
+    idx = np.sort(np.random.default_rng(seed).choice(bev.shape[0] * bev.shape[1], n_pixels, replace=False)).astype(np.int32)
+    out = {"pixel_index": idx, "bev": bev.reshape(-1, 3)[idx]}
+    for n, cam in zip(NAMES, b.cameras):
+        out[f"bev_map1_{n}"] = cam.bev_maps[0].reshape(-1, 2)[idx]
+    np.savez_compressed(os.path.join(OUT, "reference_samples.npz"), **out)
 
 
 if __name__ == "__main__":

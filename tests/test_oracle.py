@@ -1,15 +1,16 @@
 """CPU tests that PIN the oracle: restatement (oracle/restate.py) == the reference's
 cv2 call sequence (oracle/cv2_path.py) == golden hashes made from the unmodified
-reference (tests/golden/golden.json) == the unmodified reference itself when
-/root/reference is present."""
+reference (tests/golden/golden.json) == values recorded from the unmodified reference
+(tests/golden/reference_samples.npz)."""
+import os
+
 import cv2
 import numpy as np
 import pytest
 
 from oracle import cv2_path as C
-from oracle import ref_loader as RL
 from oracle import restate as R
-from tests.helpers import NAMES, h16
+from tests.helpers import GOLD, NAMES, h16
 
 
 def test_fixture_decode_hashes(fx):
@@ -140,14 +141,21 @@ def test_incalib_excalib_tools_golden(fx):
     assert h16(R.remap_linear(fx.img("front"), m1, m2)) == fx.gold["tools_undistort_front"]
 
 
-@pytest.mark.skipif(not RL.available(), reason="/root/reference not present (GPU box)")
 def test_live_unmodified_reference(fx):
-    """The unmodified reference classes, imported in place, agree with the golden file."""
-    F = fx.frames()
-    b = RL.make_bev(blend=True, balance=True)
-    assert h16(b(*F, fx.car())) == fx.gold["native"]["blend1_balance1"]["car"]
-    for n, cam in zip(NAMES, b.cameras):
+    """The unmodified reference's own outputs (canvas and BEV maps at seeded pixels, recorded by
+    oracle/gen_golden.py into tests/golden/reference_samples.npz) agree with the oracle, whose full outputs
+    agree with the golden file."""
+    z = np.load(os.path.join(GOLD, "reference_samples.npz"))
+    idx = z["pixel_index"]
+    g = fx.geometry()
+    masks = [R.blend_mask(n, g.BW, g.BH, g.CW, g.CH) for n in NAMES]
+    ref = C.RefBev(fx.calib, g, True, True, masks=masks)
+    out = ref(*fx.frames(), fx.car())
+    assert h16(out) == fx.gold["native"]["blend1_balance1"]["car"]
+    assert (out.reshape(-1, 3)[idx] == z["bev"]).all()
+    for n, cam in zip(NAMES, ref.cameras):
         assert h16(cam.bev_maps[0]) == fx.gold["camera"][n]["bev_map1"]
+        assert (cam.bev_maps[0].reshape(-1, 2)[idx] == z[f"bev_map1_{n}"]).all(), n
 
 
 def test_blend_weight_integer_identity_exhaustive():
