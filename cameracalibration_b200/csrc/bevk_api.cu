@@ -1,6 +1,8 @@
 // bevk_api.cu -- C ABI of libbevk.so (see include/bevk.h) over the sm_100a kernels.
 // Host side: argument checks, 3x3 inverses the way OpenCV computes them, device
 // buffer management, the tile-plan compiler, stream ordering.  No CPU fallback.
+// Environment: BEVK_TMA=0 (read at bevk_bev_finalize) builds no TMA plan, so every call takes the gather kernel k_bev --
+// the reference the GPU tests compare k_bev_tma with; BEVK_TRACE_FILE (-DBEVK_TRACE builds only) receives a slot timeline.
 #include <cuda.h>
 #include <cuda_runtime.h>
 
@@ -29,22 +31,6 @@
 #include <nvtx3/nvToolsExt.h>   // header-only: ranges cost nothing unless a profiler injects itself
 
 using namespace bevk;
-
-// k_bev_tma configurations built into the library: FS = bytes of one frame-set's staged source box (a ring slot holds 4 FS
-// of boxes), STAGES = ring slots, MINCTAS = resident CTAs per SM the register budget is set for, EG = LUT-entry groups per
-// slot (the plan's items never span more).  The first entry is the default; BEVK_TMA_CFG="<FS>,<STAGES>,<EG>" (read at
-// bevk_bev_finalize) selects another one for tuning runs.  Measured on B200 (profiles/r02_*stage_sweep*): with two CTAs per
-// SM the largest slots that fit win (fewer, fuller slots: 0.121 ms at FS 4096 -> 0.109 ms at FS 7936); a third, smaller
-// stage does not pay.  7936: 2 x (2 x 48256 + 16896 + 1056) + static/reserved = 233024 of the SM's 233472 bytes.
-#define BEVK_TMA_CONFIGS(X) X(7936, 2, 2, 4) X(7680, 2, 2, 4) X(6144, 2, 2, 4) X(5120, 2, 2, 4) X(4096, 2, 2, 4) X(4096, 3, 2, 2) X(4096, 2, 3, 2)
-struct TmaConfig { int fs, stages, min_ctas, eg; };
-#define X(FS, ST, MC, EG) {FS, ST, MC, EG},
-static const TmaConfig kTmaConfigs[] = {BEVK_TMA_CONFIGS(X)};
-#undef X
-static const int kNumTmaConfigs = (int)(sizeof kTmaConfigs / sizeof kTmaConfigs[0]);
-constexpr int kMaxTmaConfigs = 8;   // bevk_ctx::tma_grid
-static_assert(sizeof kTmaConfigs / sizeof kTmaConfigs[0] <= kMaxTmaConfigs, "grow bevk_ctx::tma_grid");
-
 
 // ------------------------------------------------------------------ errors
 static thread_local std::string g_err;
@@ -144,18 +130,15 @@ struct bevk_ctx {
   BevCam cam[BEVK_MAX_CAMERAS];
   bool planned = false;
   long long n_tiles = 0, n_items = 0, span_px = 0;
-  int nb_override = 0;   // BEVK_NB tuning override, read at finalize
   int bev_interp = BEVK_INTER_LINEAR;   // cv2.remap interpolation the BEV LUT is compiled for
-  int n_bands = 1;
-  bool zero_copy_ok = true;                 // BEVK_ZEROCOPY=0 forces the DMA path
   DevBuf d_hptrs;                           // device copy of the mapped host frame pointers (per half)
   const uint8_t** h_hptrs = nullptr;        // pinned staging of those pointers
   cudaEvent_t ev_hp[2] = {nullptr, nullptr};
   long long span_fetch_bytes = 0;           // bytes k_fetch_spans moves per frame-set
   long long last_h2d_bytes = 0;             // host->device bytes of the last bevk_bev_run call
-  int cam_box[BEVK_MAX_CAMERAS][BEVK_MAX_BANDS][4] = {};   // per camera and band: sampled rows [y0,y1), bytes [bx0,bx1)
+  int cam_box[BEVK_MAX_CAMERAS][DMA_BANDS][4] = {};   // per camera and band: sampled rows [y0,y1), bytes [bx0,bx1)
   DevBuf d_tiles, d_items, d_lut, d_hsv;
-  int bev_grid[6] = {0, 0, 0, 0, 0, 0};   // resident CTAs of k_bev<BAL, NB>: index = 3*BAL + {NB=1:0, 4:1, 8:2}
+  int bev_grid[4] = {0, 0, 0, 0};         // resident CTAs of k_bev<BAL, NB>: index = 2*BAL + {NB=1:0, 4:1}
   DevBuf d_frames, d_ptrs, d_canvas, d_car, d_vsum, d_delta, d_csum;
   DevBuf d_spans, d_bal, d_bal_ptrs;        // BALANCE: sampled row spans per camera, balanced frame copies + their table
   const void* bal_ptrs_for = nullptr; long long bal_ptrs_n = 0; size_t bal_ptrs_pad = 0;
@@ -163,16 +146,13 @@ struct bevk_ctx {
   std::vector<const void*> user_tab;        // ... and what it currently holds
   // TMA-staged kernel (bevk_bev_tma.cuh): its plan, and the tensor maps of the frame stacks seen recently
   bool tma_planned = false;
-  int tma_stage_bytes = 0;
   long long tma_items = 0, tma_box_bytes = 0, tma_entries = 0, tma_gather_entries = 0;
   std::vector<int2> tma_shapes;
   DevBuf d_ttiles, d_titems, d_tlut, d_unit_counter;
   struct MapSet { const void* base = nullptr; long long stride = 0, frames = 0; DevBuf d; unsigned long long used = 0; };
   MapSet maps[4];
   unsigned long long map_clock = 0;
-  int tma_cfg = 0;                          // index into kTmaConfigs
-  int tma_backoff_ns = 0;                   // BEVK_TMA_BACKOFF (read at finalize): producer poll interval when the ring is full
-  int tma_grid[kMaxTmaConfigs][4] = {};                  // [config] resident CTAs of k_bev_tma<BAL, NB>: index = 2*BAL + {NB=1:0, 4:1}
+  int tma_grid[4] = {};                     // resident CTAs of k_bev_tma<BAL, NB>: index = 2*BAL + {NB=1:0, 4:1}
   DevBuf d_stack_ptrs;                      // pointer table of a frame stack (BALANCE pre-passes read frames through a table)
   const void* stack_ptrs_base = nullptr; long long stack_ptrs_stride = 0, stack_ptrs_n = 0;
   int last_path = 0;                        // 1: k_bev (pointer-table gather), 2: k_bev_tma
@@ -616,19 +596,10 @@ int bevk_blend_masks(bevk_ctx* c, const uint8_t* polys, const int32_t* lines, in
   return BEVK_OK;
 }
 
-// the instantiations of one k_bev_tma configuration: {BAL=0,NB=1}, {0,4}, {1,1}, {1,4}, and the peer-store forms of the first two
-struct TmaFns { const void* fn[6]; };
-static TmaFns tma_fns(int cfg) {
-  int i = 0;
-#define X(FS, ST, MC, EG)                                                                                              \
-  if (i++ == cfg)                                                                                                      \
-    return TmaFns{{(const void*)k_bev_tma<false, 1, FS, ST, MC, EG>, (const void*)k_bev_tma<false, 4, FS, ST, MC, EG>,   \
-                   (const void*)k_bev_tma<true, 1, FS, ST, MC, EG>, (const void*)k_bev_tma<true, 4, FS, ST, MC, EG>,     \
-                   (const void*)k_bev_tma<false, 1, FS, ST, MC, EG, true>, (const void*)k_bev_tma<false, 4, FS, ST, MC, EG, true>}};
-  BEVK_TMA_CONFIGS(X)
-#undef X
-  return TmaFns{{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}};
-}
+// the instantiations of k_bev_tma: {BAL=0,NB=1}, {0,4}, {1,1}, {1,4}, and the peer-store forms of the first two
+static const void* const kTmaFns[6] = {(const void*)k_bev_tma<false, 1>, (const void*)k_bev_tma<false, 4>,
+                                       (const void*)k_bev_tma<true, 1>, (const void*)k_bev_tma<true, 4>,
+                                       (const void*)k_bev_tma<false, 1, true>, (const void*)k_bev_tma<false, 4, true>};
 
 // Tile-plan compiler: LUT maps + masks -> per-tile item lists and thread-ordered LUT blocks.
 int bevk_bev_finalize(bevk_ctx* c) {
@@ -647,11 +618,6 @@ int bevk_bev_finalize(bevk_ctx* c) {
     CU(cudaMemcpyAsync(m2[k].data(), c->cam[k].map2.p, npx * 2, cudaMemcpyDeviceToHost, c->stream));
   }
   CU(cudaStreamSynchronize(c->stream));
-  c->nb_override = 0;
-  if (const char* env = getenv("BEVK_NB")) {   // tuning override of the frame-sets per work unit: 1, 4 or 8
-    const int v = atoi(env);
-    if (v == 1 || v == 4 || v == 8) c->nb_override = v;
-  }
   BevPlan plan;
   {
     std::vector<const short*> p1(NC);
@@ -680,14 +646,10 @@ int bevk_bev_finalize(bevk_ctx* c) {
   for (const auto& sp : spans) c->span_px += sp.y - sp.x;
   // Host-path ingest: page-locked frames are read span by span (k_fetch_spans), pageable ones as a few DMA
   // rectangles per frame (plan_bands); BALANCE needs whole frames (its V means cover them).
-  c->zero_copy_ok = true;
-  if (const char* env = getenv("BEVK_ZEROCOPY")) c->zero_copy_ok = atoi(env) != 0;
   c->span_fetch_bytes = 0;
   for (const auto& sp : spans)
     if (sp.y > sp.x) c->span_fetch_bytes += std::min<int>(FW * 3, (3 * sp.y + 12 + 15) & ~15) - (std::max(0, 3 * sp.x - 12) & ~15);
-  c->n_bands = 2;
-  if (const char* env = getenv("BEVK_BANDS")) c->n_bands = std::max(1, std::min(BEVK_MAX_BANDS, atoi(env)));
-  for (int k = 0; k < NC; ++k) plan_bands(spans.data() + (size_t)k * FH, FW, FH, c->n_bands, c->cam_box[k]);
+  for (int k = 0; k < NC; ++k) plan_bands(spans.data() + (size_t)k * FH, FW, FH, c->cam_box[k]);
   // OpenCV's 8-bit HSV division tables (color_hsv: sdiv_table / hdiv_table180, hsv_shift = 12)
   std::vector<int> tab(512, 0);
   for (int i = 1; i < 256; ++i) {
@@ -699,16 +661,6 @@ int bevk_bev_finalize(bevk_ctx* c) {
   CU(cudaStreamSynchronize(c->stream));
   // ---- the TMA-staged kernel's plan (frames whose row pitch is a multiple of 16 bytes)
   c->tma_planned = false;
-  c->tma_cfg = 0;
-  if (const char* env = getenv("BEVK_TMA_CFG")) {
-    int fs = 0, st = 0, eg = 0;
-    if (sscanf(env, "%d,%d,%d", &fs, &st, &eg) == 3)
-      for (int i = 0; i < kNumTmaConfigs; ++i)
-        if (kTmaConfigs[i].fs == fs && kTmaConfigs[i].stages == st && kTmaConfigs[i].eg == eg) c->tma_cfg = i;
-  }
-  c->tma_stage_bytes = kTmaConfigs[c->tma_cfg].fs;
-  c->tma_backoff_ns = 0;
-  if (const char* env = getenv("BEVK_TMA_BACKOFF")) c->tma_backoff_ns = std::max(0, atoi(env));
   {
     TmaPlan tp;
     std::vector<const short*> p1(NC);
@@ -718,9 +670,7 @@ int bevk_bev_finalize(bevk_ctx* c) {
     const char* env = getenv("BEVK_TMA");
     const bool want = !(env && atoi(env) == 0) && ((unsigned)FW * 3u) % 16u == 0;
     if (want) {
-      const char* mm = getenv("BEVK_TMA_MAXMULT");   // tuning: largest multi-pass box (1, 2 or 4 FS); larger boxes become GATHER items
-      build_tma_plan(NC, FW, FH, BW, BH, c->bev_interp == BEVK_INTER_NEAREST, p1.data(), p2.data(), pm.data(), c->tma_stage_bytes, true, tp,
-                     kTmaConfigs[c->tma_cfg].eg, mm ? std::max(1, std::min(4, atoi(mm))) : 4);
+      build_tma_plan(NC, FW, FH, BW, BH, c->bev_interp == BEVK_INTER_NEAREST, p1.data(), p2.data(), pm.data(), TMA_FS, true, tp);
       RET(c->d_ttiles.ensure(tp.tiles.size() * sizeof(int4)));
       RET(c->d_titems.ensure(std::max<size_t>(1, tp.items.size()) * sizeof(TmaItem)));
       RET(c->d_tlut.ensure(std::max<size_t>(1, tp.lut.size()) * sizeof(uint4)));
@@ -737,30 +687,27 @@ int bevk_bev_finalize(bevk_ctx* c) {
       c->tma_planned = true;
     }
   }
-  if (c->tma_planned && c->tma_grid[c->tma_cfg][0] == 0) {
+  if (c->tma_planned && c->tma_grid[0] == 0) {
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, c->device));
-    const TmaFns f = tma_fns(c->tma_cfg);
-    const int nb[6] = {1, 4, 1, 4, 1, 4};
     for (int i = 0; i < 6; ++i) {
       int per_sm = 0;
-      const size_t smem = bev_tma_smem_bytes(nb[i], kTmaConfigs[c->tma_cfg].fs, kTmaConfigs[c->tma_cfg].stages, kTmaConfigs[c->tma_cfg].eg);
-      CU(cudaFuncSetAttribute(f.fn[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      // two CTAs of the default configuration fill the SM's shared memory to within 448 bytes: ask for the full carve-out
-      CU(cudaFuncSetAttribute(f.fn[i], cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, f.fn[i], TMA_THREADS, smem));
-      if (i < 4) c->tma_grid[c->tma_cfg][i] = std::max(1, per_sm) * prop.multiProcessorCount;
+      const size_t smem = bev_tma_smem_bytes(i % 2 ? 4 : 1);
+      CU(cudaFuncSetAttribute(kTmaFns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      // two CTAs fill the SM's shared memory to within 448 bytes: ask for the full carve-out
+      CU(cudaFuncSetAttribute(kTmaFns[i], cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kTmaFns[i], TMA_THREADS, smem));
+      if (i < 4) c->tma_grid[i] = std::max(1, per_sm) * prop.multiProcessorCount;
     }
   }
   if (c->bev_grid[0] == 0) {   // persistent grid = resident CTAs of each variant
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, c->device));
-    const void* fn[6] = {(const void*)k_bev<false, 1>, (const void*)k_bev<false, 4>, (const void*)k_bev<false, 8>,
-                         (const void*)k_bev<true, 1>, (const void*)k_bev<true, 4>, (const void*)k_bev<true, 8>};
-    const int nb[6] = {1, 4, 8, 1, 4, 8};
-    for (int i = 0; i < 6; ++i) {
+    const void* fn[4] = {(const void*)k_bev<false, 1>, (const void*)k_bev<false, 4>, (const void*)k_bev<true, 1>,
+                         (const void*)k_bev<true, 4>};
+    for (int i = 0; i < 4; ++i) {
       int per_sm = 0;
-      const size_t smem = bev_smem_bytes(i >= 3, nb[i]);
+      const size_t smem = bev_smem_bytes(i >= 2, i % 2 ? 4 : 1);
       CU(cudaFuncSetAttribute(fn[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn[i], 256, smem));
       c->bev_grid[i] = std::max(1, per_sm) * prop.multiProcessorCount;
@@ -801,7 +748,7 @@ int bevk_bev_host_copy_bytes(bevk_ctx* c, int flags, int64_t* h2d, int64_t* d2h)
   int64_t up = 0;
   for (int k = 0; k < c->n_cam; ++k) {
     if (flags & BEVK_FLAG_BALANCE) { up += (int64_t)c->FW * c->FH * 3; continue; }
-    for (int bnd = 0; bnd < c->n_bands; ++bnd)
+    for (int bnd = 0; bnd < DMA_BANDS; ++bnd)
       up += (int64_t)(c->cam_box[k][bnd][1] - c->cam_box[k][bnd][0]) * (c->cam_box[k][bnd][3] - c->cam_box[k][bnd][2]);
   }
   if (h2d) *h2d = up;
@@ -888,9 +835,8 @@ static int stack_table(bevk_ctx* c, const uint8_t* base, long long stride, int n
 static int launch_bev_tma(bevk_ctx* c, const TmaParams& P, int nbu, bool bal) {
   const long long units = c->n_tiles * ((P.batch + nbu - 1) / nbu);
   const int variant = (bal ? 2 : 0) + (nbu == 4 ? 1 : 0);
-  const TmaConfig cfg = kTmaConfigs[c->tma_cfg];
-  const unsigned blocks = (unsigned)std::max<long long>(1, std::min<long long>(units, c->tma_grid[c->tma_cfg][variant]));
-  const size_t smem = bev_tma_smem_bytes(nbu, cfg.fs, cfg.stages, cfg.eg);
+  const unsigned blocks = (unsigned)std::max<long long>(1, std::min<long long>(units, c->tma_grid[variant]));
+  const size_t smem = bev_tma_smem_bytes(nbu);
   const bool scatter = P.world != 0;   // peer-store output: only without BALANCE (run_device checks)
 #ifdef BEVK_TRACE
   // slot timeline (tools/gpu/trace_slots.py): the 12th launch of the process records clock64 stamps of the first 8 CTAs
@@ -908,7 +854,7 @@ static int launch_bev_tma(bevk_ctx* c, const TmaParams& P, int nbu, bool bal) {
 #else
   void* args[] = {const_cast<TmaParams*>(&P)};
 #endif
-  CU(cudaLaunchKernel(tma_fns(c->tma_cfg).fn[scatter ? 4 + (nbu == 4 ? 1 : 0) : variant], dim3(blocks), dim3(TMA_THREADS), args, smem, c->stream));
+  CU(cudaLaunchKernel(kTmaFns[scatter ? 4 + (nbu == 4 ? 1 : 0) : variant], dim3(blocks), dim3(TMA_THREADS), args, smem, c->stream));
   LAUNCHED(c);
 #ifdef BEVK_TRACE
   if (trace_file && n_launch == 12) {
@@ -952,8 +898,7 @@ static int run_device(bevk_ctx* c, FrameSrc src, int batch, const void* d_car, i
   P.cam_lo = cam_lo; P.cam_hi = cam_hi;
   P.n_tiles = (int)c->n_tiles; P.batch = batch;
   // frame-sets per work unit: 4 amortises the LUT decode over a batch; 1 for single frames
-  int nbu = batch >= 4 ? 4 : 1;
-  if (c->nb_override) nbu = c->nb_override;
+  const int nbu = batch >= 4 ? 4 : 1;
   if (c->timed && !c->capturing) CU(cudaEventRecord(c->ev0, c->stream));
   FrameSrc gsrc = src;                         // what the fused gather reads
   if (bal) {
@@ -990,7 +935,7 @@ static int run_device(bevk_ctx* c, FrameSrc src, int batch, const void* d_car, i
   }
   // TMA-staged kernel for frame stacks (16-byte aligned base and stride); pointer-table gather otherwise
   const bool use_tma = c->tma_planned && gsrc.base && (reinterpret_cast<uintptr_t>(gsrc.base) & 15) == 0 && (gsrc.stride & 15) == 0 &&
-                       gsrc.stride >= (long long)P.pitch * c->FH && (nbu == 1 || nbu == 4);
+                       gsrc.stride >= (long long)P.pitch * c->FH;
   if (use_tma) {
     TmaParams T{};
     RET(stack_maps(c, gsrc.base, gsrc.stride, nf, &T.maps));
@@ -1000,7 +945,6 @@ static int run_device(bevk_ctx* c, FrameSrc src, int batch, const void* d_car, i
     T.n_tiles = P.n_tiles; T.batch = batch; T.out = P.out; T.BW = P.BW; T.BH = P.BH; T.canvas_bytes = P.canvas_bytes;
     T.car = P.car; T.csum = P.csum; T.cam_lo = cam_lo; T.cam_hi = cam_hi;
     T.out_pitch = P.out_pitch; T.ox = P.ox; T.oy = P.oy; T.ox1 = P.ox1; T.oy1 = P.oy1;
-    T.backoff_ns = c->tma_backoff_ns;
     if (win && win->world) { for (int r = 0; r < SHARD_MAX_RANKS; ++r) T.peer[r] = win->peer[r]; T.world = win->world; T.src_off = win->src_off; }
     RET(c->d_unit_counter.ensure(256));
     CU(cudaMemsetAsync(c->d_unit_counter.p, 0, 4, c->stream));
@@ -1012,16 +956,14 @@ static int run_device(bevk_ctx* c, FrameSrc src, int batch, const void* d_car, i
     if (!gsrc.table) RET(stack_table(c, gsrc.base, gsrc.stride, nf, &gsrc.table));
     P.srcs = reinterpret_cast<const uint8_t* const*>(gsrc.table);
     const long long units = c->n_tiles * ((batch + nbu - 1) / nbu);
-    const int variant = (bal ? 3 : 0) + (nbu == 8 ? 2 : (nbu == 4 ? 1 : 0));
+    const int variant = (bal ? 2 : 0) + (nbu == 4 ? 1 : 0);
     const unsigned bev_blocks = (unsigned)std::max<long long>(1, std::min<long long>(units, c->bev_grid[variant]));
     const size_t bev_smem = bev_smem_bytes(bal, nbu);
     if (bal) {
-      if (nbu == 8) k_bev<true, 8><<<bev_blocks, 256, bev_smem, c->stream>>>(P);
-      else if (nbu == 4) k_bev<true, 4><<<bev_blocks, 256, bev_smem, c->stream>>>(P);
+      if (nbu == 4) k_bev<true, 4><<<bev_blocks, 256, bev_smem, c->stream>>>(P);
       else k_bev<true, 1><<<bev_blocks, 256, bev_smem, c->stream>>>(P);
     } else {
-      if (nbu == 8) k_bev<false, 8><<<bev_blocks, 256, bev_smem, c->stream>>>(P);
-      else if (nbu == 4) k_bev<false, 4><<<bev_blocks, 256, bev_smem, c->stream>>>(P);
+      if (nbu == 4) k_bev<false, 4><<<bev_blocks, 256, bev_smem, c->stream>>>(P);
       else k_bev<false, 1><<<bev_blocks, 256, bev_smem, c->stream>>>(P);
     }
     LAUNCHED(c);
@@ -1133,6 +1075,11 @@ int bevk_sat_sum_device(bevk_ctx* c, const void* const* parts, int n, uint64_t b
   return BEVK_OK;
 }
 
+// Frame-sets per chunk of the host pipeline: 4 = one kernel work unit; finer chunks shorten pipeline fill / drain.
+// Measured end to end on 1x B200 at the bench workload (power limit not recorded; profiles/r01_e2e_probe.txt): chunk 4
+// 4.295 ms, 2 4.313 ms, 8 4.598 ms per 32 frame-sets.
+constexpr int kHostChunk = 4;
+
 int bevk_bev_run(bevk_ctx* c, const uint8_t* const* srcs, int64_t src_stride, int batch, const uint8_t* car, int flags,
                  uint8_t* out) {
   NvtxRange nvtx_call("bevk_bev_run (host frames -> host canvases)");
@@ -1146,8 +1093,7 @@ int bevk_bev_run(bevk_ctx* c, const uint8_t* const* srcs, int64_t src_stride, in
   // Two-deep pipeline over chunks of frame-sets: the H2D copies of chunk i+1 run on the copy
   // stream while chunk i is rendered and its canvases go back on the main stream, so the two
   // PCIe directions overlap and the kernel hides under the copies.
-  int chunk = std::min(batch, 4);   // 4 frame-sets = one kernel work group; finer chunks shorten pipeline fill / drain
-  if (const char* env = getenv("BEVK_CHUNK")) chunk = std::max(1, std::min(std::min(batch, 8), atoi(env)));
+  const int chunk = std::min(batch, kHostChunk);
   const size_t set_frames = (size_t)c->n_cam;
   RET(c->d_frames.ensure(fpad * set_frames * chunk * 2));
   RET(c->d_ptrs.ensure(sizeof(void*) * set_frames * chunk * 2));
@@ -1177,8 +1123,9 @@ int bevk_bev_run(bevk_ctx* c, const uint8_t* const* srcs, int64_t src_stride, in
   CU(cudaEventRecord(c->ev_free[1], c->stream));
   int half = 0;
   // Page-locked host frames whose rows are 16-byte friendly are ingested by k_fetch_spans (the SMs read
-  // only the sampled row spans over PCIe); anything else goes through DMA copies.
-  bool zero_copy = !(flags & BEVK_FLAG_BALANCE) && (row % 16 == 0) && (src_stride % 16 == 0) && c->zero_copy_ok;
+  // only the sampled row spans over PCIe); anything else goes through DMA copies (at the bench workload, 1x B200:
+  // 4.295 ms per 32 frame-sets zero-copy vs 6.245 ms with DMA bands for every camera, profiles/r01_e2e_probe.txt).
+  bool zero_copy = !(flags & BEVK_FLAG_BALANCE) && (row % 16 == 0) && (src_stride % 16 == 0);
   std::vector<const uint8_t*> dev_view((size_t)batch * c->n_cam, nullptr);
   if (zero_copy) {
     for (size_t i = 0; i < dev_view.size() && zero_copy; ++i) {
@@ -1194,7 +1141,7 @@ int bevk_bev_run(bevk_ctx* c, const uint8_t* const* srcs, int64_t src_stride, in
   }
   if (zero_copy) {
     RET(c->d_hptrs.ensure(sizeof(void*) * set_frames * chunk * 2));
-    if (!c->h_hptrs) CU(cudaHostAlloc(reinterpret_cast<void**>(&c->h_hptrs), sizeof(void*) * BEVK_MAX_CAMERAS * 8 * 2, cudaHostAllocDefault));
+    if (!c->h_hptrs) CU(cudaHostAlloc(reinterpret_cast<void**>(&c->h_hptrs), sizeof(void*) * BEVK_MAX_CAMERAS * kHostChunk * 2, cudaHostAllocDefault));
   }
   c->last_h2d_bytes = 0;
   for (int b0 = 0; b0 < batch; b0 += chunk, half ^= 1) {
@@ -1225,7 +1172,7 @@ int bevk_bev_run(bevk_ctx* c, const uint8_t* const* srcs, int64_t src_stride, in
         else CU(cudaMemcpy2DAsync(d, row, s, (size_t)src_stride, row, c->FH, cudaMemcpyHostToDevice, c->copy_stream));
         c->last_h2d_bytes += (long long)fbytes;
       } else {                           // only the rectangle of the frame this camera's LUT can sample
-        for (int bnd = 0; bnd < c->n_bands; ++bnd) {
+        for (int bnd = 0; bnd < DMA_BANDS; ++bnd) {
           const int* bx = c->cam_box[i % c->n_cam][bnd];
           if (bx[1] > bx[0]) {
             CU(cudaMemcpy2DAsync(d + (size_t)bx[0] * row + bx[2], row, s + (size_t)bx[0] * src_stride + bx[2],

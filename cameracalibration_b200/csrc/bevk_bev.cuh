@@ -146,7 +146,7 @@ __host__ __device__ __forceinline__ unsigned sat_add_bgr(unsigned a, unsigned b)
   return lo_s | (hi_s << 8);
 }
 
-// NB = frame-sets per work unit (1 for single-frame latency, 4/8 for batches).
+// NB = frame-sets per work unit (1 for single-frame latency, 4 for batches).
 template <bool BAL, int NB>
 #ifndef BEVK_MIN_CTAS
 #define BEVK_MIN_CTAS 4

@@ -15,7 +15,7 @@
 //     eight consumer warps never touch global memory on their way: they wait for a slot, read the descriptor, the
 //     entries (LDS.128) and their taps (LDS with immediate offsets for frame-set and word; ~1.4 bank wavefronts per
 //     load instead of 4.4 L1 tag look-ups per global load, profiles/) from shared memory, and release the slot through
-//     a second mbarrier.  Every latency of the global side is the producer's, which runs STAGES slots ahead;
+//     a second mbarrier.  Every latency of the global side is the producer's, which runs TMA_STAGES slots ahead;
 //   * a stage holds 4 FS bytes: the boxes of four frame-sets of FS bytes each, or -- for the heavily minified near
 //     field, where 256 samples need 12-24 KB of source -- two boxes of 2 FS or one of 4 FS; such items take 2 or 4
 //     PASSES over their entries, one ring slot per pass.  Only what does not even fit 4 FS (discontinuities of the
@@ -42,6 +42,23 @@ constexpr unsigned T_ACTIVE = 1u << 29, T_SLOW = 1u << 30 /* GATHER entries */, 
 constexpr int ITEM_GATHER = 1, ITEM_NOSAT = 2, ITEM_FULL = 4;
 constexpr int TMA_CONSUMERS = 256, TMA_THREADS = TMA_CONSUMERS + 32;
 constexpr int TMA_DESC_BYTES = 128;   // sizeof(CUtensorMap)
+
+// The one configuration of k_bev_tma.  Every value won a measurement on 1x B200 at the bench workload (power limit not
+// recorded; profiles/r02_k_bev_tma_ab_runs.txt §3, experiments/README.md):
+//   TMA_FS        bytes of one frame-set's staged source box; a ring slot holds 4 FS of boxes.  With two CTAs per SM the
+//                 largest slots that fit win (fewer, fuller slots: 0.121 ms at FS 4096 -> 0.109 ms at FS 7936).  7936:
+//                 2 x (2 x 48256 + 16896 + 1056) + static/reserved = 233024 of the SM's 233472 bytes.
+//   TMA_STAGES    ring slots: a third, smaller slot does not pay (three slots of FS 4096 / 5120: 0.121 / 0.120 ms).
+//   TMA_MIN_CTAS  resident CTAs per SM the register budget (96) is set for: 3 CTAs/SM at 72 registers measured 0.18 vs
+//                 0.14 ms (the spills land in the item loop).
+//   TMA_EG        LUT-entry groups a slot holds, i.e. all four of a block (the plan's items never span more).
+constexpr int TMA_FS = 7936, TMA_STAGES = 2, TMA_MIN_CTAS = 2, TMA_EG = 4;
+// ring slot: boxes (4 FS) | LUT entries of up to EG groups (EG * 4 KB) | descriptor (128 B reserved); a multiple of 128:
+// TMA destinations
+constexpr int TMA_SLOT_BYTES = 4 * TMA_FS + TMA_EG * 4096 + 128;
+constexpr size_t bev_tma_smem_bytes(int nb) {
+  return (size_t)TMA_STAGES * TMA_SLOT_BYTES + (size_t)nb * ACC_WORDS * 4 + (size_t)TMA_STAGES * 16 + 1024;   // + alignment slack
+}
 
 struct __align__(16) TmaItem {   // 32 B, read as two 16-byte words
   int lut_block;                 // LUT block of this (tile, camera): entries [lut_block*1024, +1024)
@@ -72,7 +89,6 @@ struct TmaParams {
   // output window (camera-sharded runs render only the tile-aligned bounding box of their cameras' masks, a "slab"):
   // canvas pixels [ox,ox1) x [oy,oy1) go to out + (y-oy)*out_pitch + (x-ox)*3; the full canvas is 0,0,BW,BH, pitch 3*BW
   int out_pitch, ox, oy, ox1, oy1;
-  int backoff_ns;                // producer poll interval while the ring is full (0: spin)
   unsigned* unit_counter;        // zeroed before the launch: next unit to hand out
   // camera-sharded runs with peer stores (bevk_bev_run_scattered): the output of frame-set b goes straight into the memory
   // of the rank that owns b -- peer[b % world] + src_off + (b / world) * canvas_bytes -- over NVLink; world == 0: plain `out`
@@ -161,18 +177,6 @@ __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
       "bra W_%=;\n\t"
       "D_%=:\n\t}" ::"r"(bar), "r"(parity), "r"(20000u) : "memory");
 }
-// producer-side wait: one thread per CTA polls; back off between polls so that it does not take issue slots from the
-// eight consumer warps of its own and the neighbouring CTAs (profiles/r02_b: 3.4 M polls per launch without it)
-__device__ __forceinline__ void mbar_wait_backoff(unsigned bar, unsigned parity, int ns) {
-  if (ns <= 0) { mbar_wait(bar, parity); return; }
-  unsigned done = 0;
-  while (true) {
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    if (done) break;
-    __nanosleep(ns);
-  }
-}
 __device__ __forceinline__ void tma_load_3d(unsigned dst, const void* map, int x, int y, int z, unsigned bar) {
   asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
                ::"r"(dst), "l"(map), "r"(x), "r"(y), "r"(z), "r"(bar) : "memory");
@@ -209,12 +213,6 @@ __device__ __forceinline__ bool elect_one() {
   return p != 0;
 }
 __device__ __forceinline__ void consumer_sync() { asm volatile("bar.sync 1, %0;" ::"n"(TMA_CONSUMERS) : "memory"); }
-
-// ring slot: boxes (4 FS) | LUT entries of up to EG groups (EG * 4 KB) | descriptor (128 B reserved)
-__host__ __device__ constexpr int slot_bytes(int fs, int eg) { return 4 * fs + eg * 4096 + 128; }   // a multiple of 128: TMA destinations
-constexpr size_t bev_tma_smem_bytes(int nb, int fs, int stages, int eg) {
-  return (size_t)stages * slot_bytes(fs, eg) + (size_t)nb * ACC_WORDS * 4 + (size_t)stages * 16 + 1024;   // + alignment slack
-}
 
 // Slot descriptor: two 16-byte words written by the producer, everything pre-digested so that a consumer warp spends a
 // handful of instructions per slot.
@@ -282,7 +280,7 @@ __device__ __forceinline__ void gather_entry(const TmaParams& P, const uint4 e, 
 // TMA slots: `nk` groups of LUT entries (in the slot, `ent` = this thread's first entry) applied to NBP staged boxes.
 // RS: slot bytes between the boxes of consecutive frame-sets; `pitch`: bytes between the rows of a box.  FIRST: this
 // camera stores (zeros where its mask is 0), later cameras add; FULL: every weight of the item is 255.
-template <int NBP, int RS, bool FIRST, bool FULL, bool HALVES, bool NOSAT>
+template <int NBP, int RS, bool FIRST, bool FULL, bool NOSAT>
 __device__ __forceinline__ void tma_item(unsigned ent, int nk, unsigned sbase, unsigned pitch, unsigned aa, unsigned astep) {
   uint4 nxt = lds128(ent);
 #pragma unroll 1
@@ -299,41 +297,36 @@ __device__ __forceinline__ void tma_item(unsigned ent, int nk, unsigned sbase, u
     }
     const unsigned o0 = sbase + e.x, o1 = o0 + pitch;
     const unsigned sh = tma_entry_shift(e.w), third = e.w & T_THIRD, c = FULL ? 0u : tma_entry_round(e.w);
-    // HALVES (3 CTAs per SM configurations): two frame-sets at a time, 12 words in flight, to stay inside 72 registers
-    constexpr int G = HALVES && NBP > 2 ? 2 : NBP;
+    unsigned a0[NBP], a1[NBP], a2[NBP], b0[NBP], b1[NBP], b2[NBP];
 #pragma unroll
-    for (int h = 0; h < NBP; h += G) {
-      unsigned a0[G], a1[G], a2[G], b0[G], b1[G], b2[G];
+    for (int j = 0; j < NBP; ++j) {
+      const unsigned r0 = o0 + j * RS, r1 = o1 + j * RS;
+      a0[j] = lds32(r0); a1[j] = lds32(r0 + 4); a2[j] = lds32_if(r0 + 8, third);
+      b0[j] = lds32(r1); b1[j] = lds32(r1 + 4); b2[j] = lds32_if(r1 + 8, third);
+    }
 #pragma unroll
-      for (int j = 0; j < G; ++j) {
-        const unsigned r0 = o0 + (h + j) * RS, r1 = o1 + (h + j) * RS;
-        a0[j] = lds32(r0); a1[j] = lds32(r0 + 4); a2[j] = lds32_if(r0 + 8, third);
-        b0[j] = lds32(r1); b1[j] = lds32(r1 + 4); b2[j] = lds32_if(r1 + 8, third);
+    for (int j = 0; j < NBP; ++j) {
+      unsigned sb, sg, sr;
+      interp_sums(sh, e.y, e.z, a0[j], a1[j], a2[j], b0[j], b1[j], b2[j], sb, sg, sr);
+      unsigned v = weight_pack16<FULL>(sb, sg, sr, e.w, c);
+      if (!FIRST) {
+        const unsigned old = lds32(aa + j * ACC_WORDS * 4);
+        v = NOSAT ? v + old : sat_add_bgr(v, old);                        // cv2.add chain, reference camera order
       }
-#pragma unroll
-      for (int j = 0; j < G; ++j) {
-        unsigned sb, sg, sr;
-        interp_sums(sh, e.y, e.z, a0[j], a1[j], a2[j], b0[j], b1[j], b2[j], sb, sg, sr);
-        unsigned v = weight_pack16<FULL>(sb, sg, sr, e.w, c);
-        if (!FIRST) {
-          const unsigned old = lds32(aa + (h + j) * ACC_WORDS * 4);
-          v = NOSAT ? v + old : sat_add_bgr(v, old);                      // cv2.add chain, reference camera order
-        }
-        sts32(aa + (h + j) * ACC_WORDS * 4, v);
-      }
+      sts32(aa + j * ACC_WORDS * 4, v);
     }
   }
 }
 
 // one pass of a TMA item: NBP frame-sets whose boxes lie RS bytes apart in the slot
-template <int NBP, int RS, bool HALVES>
+template <int NBP, int RS>
 __device__ __forceinline__ void tma_pass(unsigned ent, int nk, unsigned sbase, unsigned pitch, unsigned aa, unsigned astep,
                                          unsigned flags) {
   if (!(flags & D_FIRST)) {   // NOSAT: the masks of the tile sum to <= 255 everywhere (always so for the reference's blend masks): plain add
-    if (flags & D_NOSAT) tma_item<NBP, RS, false, false, HALVES, true>(ent, nk, sbase, pitch, aa, astep);
-    else tma_item<NBP, RS, false, false, HALVES, false>(ent, nk, sbase, pitch, aa, astep);
-  } else if (NBP == 4 && (flags & D_FULL)) tma_item<NBP, RS, true, true, HALVES, true>(ent, nk, sbase, pitch, aa, astep);
-  else tma_item<NBP, RS, true, false, HALVES, true>(ent, nk, sbase, pitch, aa, astep);
+    if (flags & D_NOSAT) tma_item<NBP, RS, false, false, true>(ent, nk, sbase, pitch, aa, astep);
+    else tma_item<NBP, RS, false, false, false>(ent, nk, sbase, pitch, aa, astep);
+  } else if (NBP == 4 && (flags & D_FULL)) tma_item<NBP, RS, true, true, true>(ent, nk, sbase, pitch, aa, astep);
+  else tma_item<NBP, RS, true, false, true>(ent, nk, sbase, pitch, aa, astep);
 }
 
 // where frame-set b of the call is written: the caller's buffer, or (scattered mode) the owning rank's slab buffer
@@ -364,24 +357,23 @@ __device__ __forceinline__ void tile_rows_out(const TmaParams& P, unsigned wacc,
   }
 }
 
-// EG: LUT-entry groups a ring slot can hold (the plan's items never have more)
-template <bool BAL, int NB, int FS, int STAGES, int MINCTAS, int EG, bool SCATTER = false>
-__global__ void __launch_bounds__(TMA_THREADS, MINCTAS) k_bev_tma(const TmaParams P) {
-  constexpr int SB = 4 * FS;                      // box bytes of one ring slot
-  constexpr int SLOT = slot_bytes(FS, EG);        // boxes | entries | descriptor
-  constexpr int ENT_OFF = SB, DESC_OFF = SB + EG * 4096;
+template <bool BAL, int NB, bool SCATTER = false>
+__global__ void __launch_bounds__(TMA_THREADS, TMA_MIN_CTAS) k_bev_tma(const TmaParams P) {
+  constexpr int SB = 4 * TMA_FS;                  // box bytes of one ring slot
+  constexpr int SLOT = TMA_SLOT_BYTES;            // boxes | entries | descriptor
+  constexpr int ENT_OFF = SB, DESC_OFF = SB + TMA_EG * 4096;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   // slots need 128-byte alignment for cp.async.bulk.tensor; align the base to 1024 (pointer arithmetic only, so the
   // compiler keeps the shared address space)
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  unsigned* acc = reinterpret_cast<unsigned*>(smem + (size_t)STAGES * SLOT);   // [NB][ACC_WORDS] packed BGRX
-  const unsigned bar_full = smem_u32(acc + NB * ACC_WORDS), bar_empty = bar_full + 8 * STAGES;
+  unsigned* acc = reinterpret_cast<unsigned*>(smem + (size_t)TMA_STAGES * SLOT);   // [NB][ACC_WORDS] packed BGRX
+  const unsigned bar_full = smem_u32(acc + NB * ACC_WORDS), bar_empty = bar_full + 8 * TMA_STAGES;
   const unsigned stage0 = smem_u32(smem), acc_u32 = smem_u32(acc);
   __shared__ unsigned long long s_sum[BAL ? 3 * NB : 1];
   const int t = threadIdx.x, lane = t & 31, wrp = t >> 5;
   if (BAL && t < 3 * NB) s_sum[t] = 0ull;
   if (t == 0) {
-    for (int s = 0; s < STAGES; ++s) {
+    for (int s = 0; s < TMA_STAGES; ++s) {
       mbar_init(bar_full + 8 * s, 1);                      // the producer's arrive(.expect_tx)
       mbar_init(bar_empty + 8 * s, TMA_CONSUMERS / 32);    // one arrival per consumer warp
     }
@@ -392,7 +384,7 @@ __global__ void __launch_bounds__(TMA_THREADS, MINCTAS) k_bev_tma(const TmaParam
   const long long n_units = (long long)P.n_tiles * groups;
 
   if (t >= TMA_CONSUMERS) {
-    // ---------------- producer: one thread turns the plan into ring slots and stays STAGES slots ahead of the consumers
+    // ---------------- producer: one thread turns the plan into ring slots and stays TMA_STAGES slots ahead of the consumers
     if (t == TMA_CONSUMERS) {
       unsigned s = 0, ph = 0;   // ring position: slot, phase of its barriers
 #ifdef BEVK_TRACE
@@ -406,7 +398,7 @@ __global__ void __launch_bounds__(TMA_THREADS, MINCTAS) k_bev_tma(const TmaParam
         unsigned long long* T = P.trace + ((size_t)blockIdx.x * 512 + tn) * 16;
         if (tr) T[0] = clock64();
 #endif
-        mbar_wait_backoff(bar_empty + 8 * s, ph ^ 1u, P.backoff_ns);   // consumers have left this slot
+        mbar_wait(bar_empty + 8 * s, ph ^ 1u);   // consumers have left this slot
 #ifdef BEVK_TRACE
         if (tr) { T[1] = clock64(); T[6] = tx; T[7] = d0.x; }
 #endif
@@ -415,7 +407,7 @@ __global__ void __launch_bounds__(TMA_THREADS, MINCTAS) k_bev_tma(const TmaParam
         if (tx) mbar_expect_tx(full, tx); else mbar_arrive(full);
         if (ent_bytes) bulk_copy(slot + ENT_OFF, ent_src, ent_bytes, full);
         for (int j = 0; j < np; ++j) tma_load_3d(slot + j * rs, map, bx, by, z0 + j * P.n_cam, full);
-        if (++s == STAGES) { s = 0; ph ^= 1u; }
+        if (++s == TMA_STAGES) { s = 0; ph ^= 1u; }
 #ifdef BEVK_TRACE
         if (tr) T[2] = clock64();
         ++tn;
@@ -547,9 +539,9 @@ __global__ void __launch_bounds__(TMA_THREADS, MINCTAS) k_bev_tma(const TmaParam
           gather_entry<NB>(P, lds128(ent + k * 4096), aa + k * d.w, (flags & D_FIRST) != 0, (flags & D_NOSAT) != 0, frame0, set_stride, nb);
       } else {
         const unsigned kind = (flags >> 20) & 3u;
-        if (NB == 4 && kind == 0u) tma_pass<(NB == 4 ? 4 : 1), FS, (MINCTAS > 2)>(ent, nk, slot, d.y, aa, d.w, flags);
-        else if (NB == 4 && kind == 1u) tma_pass<(NB == 4 ? 2 : 1), 2 * FS, false>(ent, nk, slot, d.y, aa, d.w, flags);
-        else tma_pass<1, 0, false>(ent, nk, slot, d.y, aa, d.w, flags);
+        if (NB == 4 && kind == 0u) tma_pass<(NB == 4 ? 4 : 1), TMA_FS>(ent, nk, slot, d.y, aa, d.w, flags);
+        else if (NB == 4 && kind == 1u) tma_pass<(NB == 4 ? 2 : 1), 2 * TMA_FS>(ent, nk, slot, d.y, aa, d.w, flags);
+        else tma_pass<1, 0>(ent, nk, slot, d.y, aa, d.w, flags);
       }
     }
     // word 1 (tile, frame-sets) is needed by the slot that ends a unit; it is read before this warp releases the slot
@@ -560,7 +552,7 @@ __global__ void __launch_bounds__(TMA_THREADS, MINCTAS) k_bev_tma(const TmaParam
     if (tr) T[5] = clock64();
 #endif
     if (elect_one()) mbar_arrive(bar_empty + 8 * s);     // this warp no longer reads the slot
-    if (++s == STAGES) { s = 0; ph ^= 1u; }
+    if (++s == TMA_STAGES) { s = 0; ph ^= 1u; }
 #ifdef BEVK_TRACE
     if (tr) T[8] = clock64();
 #endif

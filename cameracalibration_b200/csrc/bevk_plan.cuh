@@ -17,8 +17,6 @@
 
 #include "bevk_bev.cuh"
 
-#define BEVK_MAX_BANDS 8
-
 namespace bevk {
 
 struct BevPlan {
@@ -118,18 +116,19 @@ inline void build_bev_plan(int NC, int FW, int FH, int BW, int BH, bool nearest,
   for (auto& sp : out.spans) if (sp.y < 0) sp = make_int2(0, 0);
 }
 
-// Sampled region of one camera as n_bands horizontal bands, each with its own byte range [bx2, bx3) over rows
+// Sampled region of one camera as DMA_BANDS horizontal bands, each with its own byte range [bx2, bx3) over rows
 // [bx0, bx1): what the host path uploads of a pageable frame.  The footprint of a fisheye camera under a BEV mask is
 // fan-shaped: two bands already cut the plain bounding box from 34 % to 23 % of the frame.
-inline void plan_bands(const int2* spans /* [FH] of one camera */, int FW, int FH, int n_bands, int (*box)[4]) {
+constexpr int DMA_BANDS = 2;
+inline void plan_bands(const int2* spans /* [FH] of one camera */, int FW, int FH, int (*box)[4]) {
   int y0 = FH, y1 = 0;
   for (int y = 0; y < FH; ++y)
     if (spans[y].y > spans[y].x) { y0 = std::min(y0, y); y1 = std::max(y1, y + 1); }
-  for (int bnd = 0; bnd < n_bands; ++bnd) {
+  for (int bnd = 0; bnd < DMA_BANDS; ++bnd) {
     int* bx = box[bnd];
     bx[0] = bx[1] = bx[2] = bx[3] = 0;
     if (y1 <= y0) continue;
-    const int ya = y0 + (int)((long long)(y1 - y0) * bnd / n_bands), yb = y0 + (int)((long long)(y1 - y0) * (bnd + 1) / n_bands);
+    const int ya = y0 + (int)((long long)(y1 - y0) * bnd / DMA_BANDS), yb = y0 + (int)((long long)(y1 - y0) * (bnd + 1) / DMA_BANDS);
     int x0 = FW, x1 = 0;
     for (int y = ya; y < yb; ++y) {
       const int2 sp = spans[y];

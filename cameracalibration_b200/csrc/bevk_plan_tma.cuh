@@ -63,9 +63,16 @@ inline int lds_wavefronts(const unsigned* word, int n) {
   return deg;
 }
 
+// Largest multi-pass box, in stages: what exceeds 4 FS becomes a GATHER item.  Measured on 1x B200 at the bench workload
+// (power limit not recorded; profiles/r02_k_bev_tma_ab_runs.txt §3): multi-pass boxes win at every stage size, at FS 7936
+// 0.1087 ms with boxes of up to 4 FS against 0.1125 ms with 2 FS.
+constexpr int TMA_MAX_MULT = 4;
+
+// stage_bytes / max_groups: TMA_FS / TMA_EG in the library; the CPU tests also compile plans for other values to force
+// strip splits, multi-pass and GATHER items
 inline void build_tma_plan(int NC, int FW, int FH, int BW, int BH, bool nearest, const short* const* m1,
                            const unsigned short* const* m2, const uint8_t* const* masks, int stage_bytes, bool allow_tma,
-                           TmaPlan& out, int max_groups = 4, int max_mult = 4) {
+                           TmaPlan& out, int max_groups = TMA_EG) {
   const unsigned pitch = (unsigned)FW * 3u;
   const long long frame_bytes = (long long)pitch * FH;
   const int tx = (BW + TILE - 1) / TILE, ty = (BH + TILE - 1) / TILE;
@@ -163,7 +170,7 @@ inline void build_tma_plan(int NC, int FW, int FH, int BW, int BH, bool nearest,
             const long long bytes = (long long)w16 * 16 * hh;
             fits = shape_ok && bytes <= stage_bytes;
             if (!fits && shape_ok && r.g1 - r.g0 == 1) {       // a single strip: give it 2 or 4 frame-set slots of the stage
-              for (int m = 2; m <= max_mult && !fits; m *= 2)
+              for (int m = 2; m <= TMA_MAX_MULT && !fits; m *= 2)
                 if (bytes <= (long long)m * stage_bytes && (long long)m * stage_bytes <= 65536) { fits = true; fs_bytes = m * stage_bytes; }
             }
           }

@@ -183,7 +183,7 @@ int64_t bevk_bev_last_h2d_bytes(bevk_ctx *ctx);
 int bevk_bev_last_path(bevk_ctx *ctx);
 /* The TMA-staged kernel's plan: work items, tensor-map box shapes, bytes one frame-set's boxes deliver, LUT entries
  * served from staged boxes / by global gathers.  All zero when the plan does not exist (row pitch not a multiple of
- * 16 bytes, or BEVK_TMA=0). */
+ * 16 bytes, or the environment variable BEVK_TMA=0 at bevk_bev_finalize, which leaves every call to k_bev). */
 int bevk_bev_tma_plan_info(bevk_ctx *ctx, int64_t *n_items, int64_t *n_shapes, int64_t *box_bytes, int64_t *tma_entries,
                            int64_t *gather_entries);
 /* ---- multi-GPU sharding: one process (one ctx) per GPU ---------------------------------------------------

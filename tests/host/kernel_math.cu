@@ -209,6 +209,8 @@ static int mode_balance() {
 }
 
 //   kernel_math bev <in.bin> <out.bin>
+//   kernel_math bevtma <in.bin> <out.bin> shipped | <stage bytes> [<entry groups per slot>]
+//       the same through the TMA plan (bevk_plan_tma.cuh) at the library's TMA_FS / TMA_EG or at other settings
 // One frame-set through the product's plan compiler (bevk_plan.cuh, the code bevk_bev_finalize runs) and a plain-loop
 // interpreter of that plan that uses the kernels' own per-entry arithmetic (interp_fast, sample_slow_core, sat_add_bgr,
 // hsv_roundtrip, lum_deltas, gray_world_gains / gain_entry).  It mirrors k_bev's work decomposition -- tile, item,
@@ -216,7 +218,7 @@ static int mode_balance() {
 // BALANCE sequence (V sums, offsets, balanced row spans, gather, channel sums, gains, car), without threads.
 // in.bin : int32 NC FW FH BW BH nearest balance has_car; per camera map1 int16[BH*BW*2], map2 uint16[BH*BW],
 //          mask u8[BH*BW]; NC frames u8[FH*FW*3]; car u8[BH*BW*3] if has_car.   out.bin: canvas u8[BH*BW*3]
-static int mode_bev(const char* in_path, const char* out_path, int tma_stage_bytes /* 0: round-1 gather plan */, int max_groups = 4) {
+static int mode_bev(const char* in_path, const char* out_path, int tma_stage_bytes /* 0: round-1 gather plan */, int max_groups = TMA_EG) {
   FILE* f = fopen(in_path, "rb");
   if (!f) return 5;
   int hd[8];
@@ -284,6 +286,7 @@ static int mode_bev(const char* in_path, const char* out_path, int tma_stage_byt
       build_tma_plan(NC, FW, FH, BW, BH, nearest != 0, p1.data(), p2.data(), pm.data(), tma_stage_bytes, true, tp, max_groups);
     }
     std::vector<uint8_t> stage((size_t)4 * tma_stage_bytes + 16, 0xEE);   // one ring slot = 4 FS
+    long long two_pass = 0, four_pass = 0, gather_items = 0;   // items by slot kind
     for (const int4& tile : tp.tiles) {
       unsigned acc[ACC_WORDS];
       for (auto& a : acc) a = 0xdeadbeefu;                 // every word must be written before the write-out reads it
@@ -293,7 +296,10 @@ static int mode_bev(const char* in_path, const char* out_path, int tma_stage_byt
         if (first_cam < 0) first_cam = item.cam;
         const bool first = item.cam == first_cam, nosat = (item.flags & ITEM_NOSAT) != 0, gather = (item.flags & ITEM_GATHER) != 0;
         const uint8_t* src = (balance ? bal : frames)[item.cam].data();
-        if (!gather) {
+        if (gather) ++gather_items;
+        else {
+          two_pass += item.fs_bytes == 2 * tma_stage_bytes;
+          four_pass += item.fs_bytes == 4 * tma_stage_bytes;
           memset(stage.data(), 0xEE, stage.size());
           const int2 shape = tp.shapes[item.shape];
           CHECK((unsigned)(shape.x * 4 * shape.y) == item.tx_bytes && (int)item.tx_bytes <= item.fs_bytes, "box bytes");
@@ -349,8 +355,9 @@ static int mode_bev(const char* in_path, const char* out_path, int tma_stage_byt
           o[0] = px & 255u; o[1] = (px >> 8) & 255u; o[2] = (px >> 16) & 255u;
         }
     }
-    printf("tma plan: tiles=%zu items=%zu shapes=%zu box_bytes=%lld tma_entries=%lld gather_entries=%lld\n", tp.tiles.size(),
-           tp.items.size(), tp.shapes.size(), tp.box_bytes, tp.tma_entries, tp.gather_entries);
+    printf("tma plan: tiles=%zu items=%zu shapes=%zu box_bytes=%lld tma_entries=%lld gather_entries=%lld two_pass=%lld four_pass=%lld "
+           "gather_items=%lld\n", tp.tiles.size(), tp.items.size(), tp.shapes.size(), tp.box_bytes, tp.tma_entries, tp.gather_entries,
+           two_pass, four_pass, gather_items);
   } else {
   // ---- the gather (k_bev)
   for (const int4& tile : plan.tiles) {
@@ -475,7 +482,8 @@ int main(int argc, char** argv) {
     return mode_gather(atoi(argv[2]), atoi(argv[3]), atoi(argv[4]), atoi(argv[5]), atoi(argv[6]), argv[7], argv[8]);
   if (argc == 4 && !strcmp(argv[1], "bev")) return mode_bev(argv[2], argv[3], 0);
   if ((argc == 5 || argc == 6) && !strcmp(argv[1], "bevtma")) {
-    const int r = mode_bev(argv[2], argv[3], atoi(argv[4]), argc == 6 ? atoi(argv[5]) : 4);
+    const bool shipped = !strcmp(argv[4], "shipped");
+    const int r = mode_bev(argv[2], argv[3], shipped ? TMA_FS : atoi(argv[4]), argc == 6 ? atoi(argv[5]) : TMA_EG);
     return r ? r : (fails ? 1 : 0);
   }
   if (argc == 2 && !strcmp(argv[1], "balance")) return mode_balance();

@@ -4,6 +4,7 @@ against the scalar definitions of cv2.remap / BlendMask / cv2.add, (b) runs the 
 (undistort_point, quantise_uv, warp_point, the closed-form 3x3 inverse) over whole maps, compared here with live cv2.
 nvcc compiles it; only host code runs (no GPU, no CUDA runtime call)."""
 import os
+import re
 import shutil
 import subprocess
 
@@ -220,16 +221,16 @@ def _bev_on_host(exe, tmp_path, fx, g, calib, masks, frames, car, balance, neare
     assert r.returncode == 0, (r.returncode, r.stdout, r.stderr)
     out = np.fromfile(tmp_path / "bev_out.bin", np.uint8).reshape(g.BH, g.BW, 3)
     # the TMA-staged kernel's plan (bevk_plan_tma.cuh) through its own interpreter: boxes modelled as the tensor copy
-    # delivers them (zeros outside the frame); several (stage size, entry groups per slot) settings: the shipped default,
-    # one that forces strip splits / multi-pass / GATHER items, three entry groups per slot (4 groups = 3 + 1), single-group
-    # items
+    # delivers them (zeros outside the frame); several (stage size, entry groups per slot) settings: the library's own
+    # (TMA_FS, TMA_EG), one that forces strip splits / multi-pass / GATHER items, three entry groups per slot
+    # (4 groups = 3 + 1), single-group items.  info: the interpreters' output, the library's setting first.
     info = r.stdout
-    for stage, max_groups in ((7936, 4), (1536, 4), (4096, 3), (6144, 1)):
-        rt = subprocess.run([exe, "bevtma", str(tmp_path / "bev_in.bin"), str(tmp_path / "bevtma_out.bin"), str(stage), str(max_groups)],
+    for setting in (["shipped"], ["1536", "4"], ["4096", "3"], ["6144", "1"]):
+        rt = subprocess.run([exe, "bevtma", str(tmp_path / "bev_in.bin"), str(tmp_path / "bevtma_out.bin"), *setting],
                             capture_output=True, text=True, timeout=600)
         assert rt.returncode == 0, (rt.returncode, rt.stdout, rt.stderr)
         out_t = np.fromfile(tmp_path / "bevtma_out.bin", np.uint8).reshape(g.BH, g.BW, 3)
-        assert (out_t == out).all(), (stage, int((out_t != out).sum()), rt.stdout)
+        assert (out_t == out).all(), (setting, int((out_t != out).sum()), rt.stdout)
         info += rt.stdout
     return out, info
 
@@ -245,6 +246,10 @@ def test_bev_path_on_the_host_native_golden(exe, tmp_path, fx, blend, balance):
     for car_key, car in (("car", fx.car()), ("nocar", None)):
         out, info = _bev_on_host(exe, tmp_path, fx, g, fx.calib, masks, fx.frames(), car, balance)
         assert h16(out) == gold[car_key], (car_key, info)
+        # the library's plan at this geometry has every slot kind of k_bev_tma -- two- and four-pass items and GATHER
+        # items -- so the GPU A/B of this geometry against the gather kernel runs all of them
+        kinds = re.search(r"two_pass=(\d+) four_pass=(\d+) gather_items=(\d+)", info)
+        assert kinds and all(int(n) > 0 for n in kinds.groups()), info
 
 
 @pytest.mark.parametrize("key,FW,FH,BW,BH,blend,balance,car", [
